@@ -2,6 +2,7 @@
 MPII 384x384, 16 joints, batch 32 per GPU, fp16) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--precision fp16|bf16|fp32]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -44,6 +45,7 @@ WASP_LAYERWISE_BYTES_C2 = 355.6e6   # SURVEY.md 8(d): layer-by-layer bytes of th
 # aspp1 302.0 + 339.7 * (0.25 + 0.44 + 0.69) + GAP 0.5 + conv1 (4 of 5 groups) 151.0
 WASP_EXECUTED_FLOPS_PER_IMG_24 = 2.0 * (302.0 + 339.7 * 1.38 + 0.5 + 151.0) * 1e6
 NET_FLOPS_PER_IMG = 68.1e9          # SURVEY.md §8(d): conv-only fwd @384^2
+DUMP_MAX_BYTES = 64 * 10 ** 6
 
 
 def parse_args():
@@ -64,7 +66,25 @@ def parse_args():
     ap.add_argument("--no-parity-mode", action="store_true", help="skip the fp32-grade mode timing")
     ap.add_argument("--train-steps", type=int, default=6)
     ap.add_argument("--train-only", action="store_true", help="print only the training sub-record (tuning runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the heat-maps of the last timed step (rank 0) to DIR/heat.npy, fp32; above %d MB only "
+                         "the first frames that fit" % (DUMP_MAX_BYTES // 10 ** 6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.train_only):
+        ap.error("--dump-outputs needs the inference timing of --impl b200 (not --train-only)")
+    return args
+
+
+def dump_outputs(out_dir: str, heat) -> None:
+    """Saves what a caller of the timed path receives (fp32 heat-maps [N, K+1, H/8, W/8]) for output-for-output
+    comparisons of two builds: inputs and weights are seeded, so equal arguments give equal inputs."""
+    import numpy as np
+    per_frame = heat[0].numel() * 4
+    heat = heat[:max(1, DUMP_MAX_BYTES // per_frame)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "heat.npy"), heat.detach().float().cpu().numpy())
 
 
 def measured_peaks():
@@ -235,17 +255,18 @@ def run_reference(args) -> int:
 # GPU arm
 # ------------------------------------------------------------------------------------------------
 def _timed_steps(fn, steps, flush):
-    """Sum of per-step CUDA-event times (ms) of fn(), L2 flushed (untimed) before every step."""
+    """Sum of per-step CUDA-event times (ms) of fn(), L2 flushed (untimed) before every step, and what the last
+    step returned."""
     import torch
     starts = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     ends = [torch.cuda.Event(enable_timing=True) for _ in range(steps)]
     for i in range(steps):
         flush.zero_()
         starts[i].record()
-        fn()
+        out = fn()
         ends[i].record()
     torch.cuda.synchronize()
-    return sum(s.elapsed_time(e) for s, e in zip(starts, ends))
+    return sum(s.elapsed_time(e) for s, e in zip(starts, ends)), out
 
 
 def parity_record(model, x_dev, heat_dev, precision, n_check=2):
@@ -396,9 +417,11 @@ def run_b200(args) -> int:
     barrier()
     sampler = ClockSampler(local)
     sampler.start()
-    dev_ms = _timed_steps(lambda: model.forward_static(x_dev), args.steps, flush)
+    dev_ms, heat_last = _timed_steps(lambda: model.forward_static(x_dev), args.steps, flush)
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, heat_last)      # plan-owned buffer: saved before the next call overwrites it
     launches = plan.launches * args.steps
     heat_timed = model.forward_static(x_dev).clone()
 
@@ -517,7 +540,7 @@ def run_b200(args) -> int:
                 m32.forward_static(x_dev)
             torch.cuda.synchronize()
             k32 = max(3, min(args.steps, 10))
-            ms32 = _timed_steps(lambda: m32.forward_static(x_dev), k32, flush) / k32
+            ms32 = _timed_steps(lambda: m32.forward_static(x_dev), k32, flush)[0] / k32
             h32 = m32.forward_static(x_dev).clone()
             p32 = parity_record(m32, x_dev, h32, "fp32")
             parity_mode = {"precision": "fp32 (bf16x3 split, fp32 accumulate)", "ms_per_step": ms32,

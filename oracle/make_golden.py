@@ -103,9 +103,31 @@ def round2_fixtures():
         print("%-32s %8.1f KB" % (fn, os.path.getsize(os.path.join(OUT, fn)) / 1024))
 
 
+def crosscheck_fixtures():
+    """The reference's own outputs for the oracle cross-checks of tests/test_oracle.py, so that they run without the
+    reference: MPII forward at 64x64 (seeds 3 and 6) and utils/evaluate.py accuracy() (seeds 21 and 22)."""
+    os.makedirs(OUT, exist_ok=True)
+    torch.set_grad_enabled(False)
+    RefUnipose, _ref_lstm, ref_eval = import_reference()
+    out = {}
+    for seed in (3, 6):
+        torch.manual_seed(0)
+        m = RefUnipose(dataset="MPII", num_classes=16).eval()
+        m.load_state_dict(O.synth_state_dict(16, seed=seed), strict=True)
+        out["heat_seed%d" % seed] = m(O.synth_input(1, 64, 64, seed=seed)).numpy()
+    for seed in (21, 22):
+        gt, pred = E.synth_eval_inputs(4, 16, 48, seed=seed)
+        for i, v in enumerate(ref_eval.accuracy(pred, gt, 0.2, 0.5, "MPII")):
+            out["accuracy_seed%d_%d" % (seed, i)] = np.asarray(v, dtype=np.float64)
+    np.savez_compressed(os.path.join(OUT, "crosscheck_mpii_64.npz"), **out)
+    print("%-32s %8.1f KB" % ("crosscheck_mpii_64.npz", os.path.getsize(os.path.join(OUT, "crosscheck_mpii_64.npz")) / 1024))
+
+
 def main():
     if "--round2" in sys.argv:
         return round2_fixtures()
+    if "--crosscheck" in sys.argv:
+        return crosscheck_fixtures()
     os.makedirs(OUT, exist_ok=True)
     torch.manual_seed(0)
     torch.set_grad_enabled(False)
@@ -165,8 +187,8 @@ def main():
         outs["heat%d" % it] = hm.numpy()
         outs["cell%d" % it] = cell.numpy()
         outs["hide%d" % it] = hide.numpy()
-        outs["trunk%d" % it] = t.numpy()
-    outs["centermap_pooled"] = mv.pool_center(cm[:, 0]).numpy()
+        # the trunk heat-maps only scale the state tolerance of the GPU test: their max-abs keeps the file under 1 MB
+        outs["trunk%d_absmax" % it] = np.float32(t.abs().max())
     np.savez_compressed(os.path.join(OUT, "video_penn_368.npz"), **outs)
 
     # ---- evaluation path: utils/evaluate.py on identical synthetic heat-maps ----

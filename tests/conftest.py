@@ -7,7 +7,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
 
 
 def _host_cpu_budget() -> int:
@@ -42,8 +41,3 @@ def pytest_collection_modifyitems(config, items):
 @pytest.fixture(scope="session")
 def golden_dir():
     return GOLDEN
-
-
-@pytest.fixture(scope="session")
-def have_reference():
-    return os.path.isdir(os.path.join(REFERENCE, "model"))

@@ -277,7 +277,7 @@ def test_video_model_vs_golden_and_batch():
         assert heat.shape == (1, 14, 46, 46) and cell.shape == (1, 15, 46, 46)
         # the ConvLSTM states are bounded by 1 while the trunk heat-maps feeding the gates reach |47|: their error
         # is the trunk's absolute error (<= 1e-3 * max|trunk|) seen through the gate convolutions
-        trunk_scale = float(np.abs(g["trunk%d" % it]).max())
+        trunk_scale = float(g["trunk%d_absmax" % it])
         for name, t in (("heat", heat), ("cell", cell), ("hide", hide)):
             got, ref = t.cpu().numpy(), g["%s%d" % (name, it)]
             r = _rel(got, ref)

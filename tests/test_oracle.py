@@ -1,9 +1,7 @@
 """CPU tests: the oracle (oracle/*.py) against the committed golden fixtures produced by the real reference
-(oracle/make_golden.py) and, when /root/reference is present, against the live reference modules."""
-import importlib.util
+(oracle/make_golden.py)."""
 import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -12,7 +10,7 @@ import torch
 from oracle import evaluate_oracle as E
 from oracle import unipose_oracle as O
 
-from conftest import GOLDEN, REFERENCE
+from conftest import GOLDEN
 
 
 def _load(name):
@@ -77,21 +75,39 @@ def test_oracle_config5_512_and_output_stride8_vs_golden():
         _close(O.unipose_forward(x8, sd8, output_stride=8).numpy(), g8["heat"])
 
 
-def test_compiled_reference_matches_oracle_when_present():
-    """oracle/_ref (the reference's own modules as byte-code, what bench.py's CPU arm times) == the oracle port."""
-    from oracle import build_ref
-    if not build_ref.have_ref():
-        pytest.skip("oracle/_ref not built (python oracle/build_ref.py needs /root/reference)")
-    RefUnipose, _, ref_eval = build_ref.import_reference()
-    m = RefUnipose(dataset="MPII", num_classes=16).eval()
-    sd = O.synth_state_dict(16, seed=6)
-    m.load_state_dict(sd, strict=True)
-    x = O.synth_input(1, 64, 64, seed=6)
+def _check_vs_crosscheck(forward, accuracy, seed, eval_seed):
+    """forward(state_dict, x) and accuracy() against the reference's own MPII 64x64 forward and accuracy() outputs,
+    stored by `oracle/make_golden.py --crosscheck`."""
+    g = _load("crosscheck_mpii_64.npz")
+    sd = O.synth_state_dict(16, seed=seed)
     with torch.no_grad():
-        _close(O.unipose_forward(x, sd).numpy(), m(x).numpy(), rtol=1e-5, atol=1e-6)
-    gt, pred = E.synth_eval_inputs(4, 16, 48, seed=22)
-    for u, v in zip(ref_eval.accuracy(pred, gt, 0.2, 0.5, "MPII"), E.accuracy(pred, gt, 0.2, 0.5, "MPII")):
-        np.testing.assert_allclose(np.asarray(u, dtype=np.float64), np.asarray(v, dtype=np.float64), rtol=0, atol=1e-12)
+        _close(forward(sd, O.synth_input(1, 64, 64, seed=seed)).numpy(), g["heat_seed%d" % seed], rtol=1e-5, atol=1e-6)
+    gt, pred = E.synth_eval_inputs(4, 16, 48, seed=eval_seed)
+    got = accuracy(pred, gt, 0.2, 0.5, "MPII")
+    assert len(got) == 6
+    for i, v in enumerate(got):
+        np.testing.assert_allclose(np.asarray(v, dtype=np.float64), g["accuracy_seed%d_%d" % (eval_seed, i)],
+                                   rtol=0, atol=1e-12)
+
+
+def _oracle_forward(sd, x):
+    return O.unipose_forward(x, sd)
+
+
+def test_oracle_and_compiled_reference_vs_crosscheck_fixture():
+    """The oracle port == the reference's outputs; so is oracle/_ref (the reference's own modules as byte-code, what
+    bench.py's CPU arm times) where `oracle/build_ref.py` has built it."""
+    from oracle import build_ref
+    _check_vs_crosscheck(_oracle_forward, E.accuracy, 6, 22)
+    if build_ref.have_ref():
+        RefUnipose, _, ref_eval = build_ref.import_reference()
+
+        def compiled_forward(sd, x):
+            m = RefUnipose(dataset="MPII", num_classes=16).eval()
+            m.load_state_dict(sd, strict=True)
+            return m(x)
+
+        _check_vs_crosscheck(compiled_forward, ref_eval.accuracy, 6, 22)
 
 
 def test_oracle_video_vs_golden():
@@ -146,29 +162,5 @@ def test_get_kpts_oracle():
     assert E.get_kpts(m) == [[int(20 * 368.0 / 46), int(10 * 368.0 / 46)], [0, int(45 * 368.0 / 46)]]
 
 
-# ---- live cross-check against the real reference (build container only) ----------------------------
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REFERENCE, "model")), reason="/root/reference not present")
-def test_oracle_vs_live_reference_modules():
-    if REFERENCE not in sys.path:
-        sys.path.insert(0, REFERENCE)
-    from model.modules.backbone import resnet
-    resnet.model_zoo.load_url = lambda *a, **k: {}
-    from model.unipose import unipose as RefUnipose
-    torch.manual_seed(0)
-    m = RefUnipose(dataset="MPII", num_classes=16).eval()
-    sd = O.synth_state_dict(16, seed=3)
-    m.load_state_dict(sd, strict=True)
-    x = O.synth_input(1, 64, 64, seed=3)
-    with torch.no_grad():
-        ref = m(x)
-        got = O.unipose_forward(x, sd)
-    _close(got.numpy(), ref.numpy(), rtol=1e-5, atol=1e-6)
-    # evaluate.py, loaded by path (importing `utils` pulls matplotlib)
-    spec = importlib.util.spec_from_file_location("ref_evaluate", os.path.join(REFERENCE, "utils", "evaluate.py"))
-    ref_eval = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_eval)
-    gt, pred = E.synth_eval_inputs(4, 16, 48, seed=21)
-    a = ref_eval.accuracy(pred, gt, 0.2, 0.5, "MPII")
-    b = E.accuracy(pred, gt, 0.2, 0.5, "MPII")
-    for u, v in zip(a, b):
-        np.testing.assert_allclose(np.asarray(u, dtype=np.float64), np.asarray(v, dtype=np.float64), rtol=0, atol=1e-12)
+def test_oracle_vs_reference_crosscheck_fixture():
+    _check_vs_crosscheck(_oracle_forward, E.accuracy, 3, 21)
