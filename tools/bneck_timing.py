@@ -54,7 +54,8 @@ for chain in (False, True):
         "chain" if chain else "layer-wise", plan.launches, tot / 5 * 1e3, len(blocks)))
 names = {0: "entry", 1: "deps", 31: "exit"}
 for b in range(3):
-    names[2 + b] = "b%d_halo_ok" % b
+    names[23 + b] = "b%d_conv2_first_mma" % b      # centre tap of chunks 0-1 issued (staged t1 tile)
+    names[26 + b] = "b%d_halo_c0_mma" % b          # first halo MMA (chunk 0) issued: counter[b][0] complete + TMA
     names[5 + b] = "b%d_conv2_issued" % b
     names[8 + b] = "b%d_p3_issued" % b
     names[11 + b] = "b%d_t2_epi_done" % b
@@ -66,7 +67,7 @@ t = np.array(buf, dtype=np.float64).reshape(160, 32)
 t = t[t[:, 0] > 0]
 t0 = t[:, 0].min()
 print("CTAs", len(t))
-order = [0, 1, 2, 5, 11, 8, 14, 17, 3, 6, 12, 9, 15, 18, 4, 7, 13, 10, 16, 19, 31]
+order = [0, 1] + [k + b for b in range(3) for k in (23, 26, 5, 11, 8, 14, 17)] + [31]
 for k in order:
     col = t[:, k]
     col = col[col > 0]

@@ -5,19 +5,40 @@
 // conv, and that is PER IMAGE, so CTAs synchronise through per-image-group release/acquire counters instead of
 // kernel boundaries.  Every CTA owns one 128-pixel tile for the whole run; CTA pairs (cta_group::2, M = 256) take the
 // same tile of two consecutive image groups.  Per block b (input X_b [.., 1024], T1_b = conv1(X_b) [.., 256]):
-//   P2  conv2 3x3:  halo tiles of T1_b by TMA (after the group's counter says every tile stored T1_b) -> acc[256]
-//       epilogue: t2 = ReLU(acc + shift2) -> 16-bit -> staging set T (never goes to global memory)
+//   P2  conv2 3x3 -> acc[256]: the centre tap first, from this CTA's own t1 tile in the staging set T, then the halo
+//       taps chunk-major over the four 64-channel chunks c of T1_b (chunk 0's eight taps, then chunk 1's, ...).  The
+//       halo tiles of chunk c are TMA-loaded once counter[b][c] says every tile of the image group stored chunk c of
+//       T1_b, so chunk 0's halo MMAs run while the neighbours are still storing chunks 1..3.
+//       epilogue: t2 = ReLU(acc + shift2) -> 16-bit -> staging set T (never goes to global memory); accumulator half
+//       0 (t2 groups 0-1) is released as soon as it is in registers, so conv3 N-tile 0 starts mid-epilogue
 //   P3  conv3 1x1 in eight N-tiles of 128 output channels, ping-pong in TMEM columns [0,128) / [128,256):
 //         acc_j = t2 (A operand straight from the staging set T) x W3_j  (+ X_b residual tile x I as identity MMAs)
+//         N-tile 0 takes K-chunk c as soon as t2 group c is staged
 //         epilogue j (overlaps the MMAs of N-tile j+1): X_{b+1}[:, j] = ReLU(acc_j + shift3) -> staging set O
 //           -> TMA store (the next block's residual) AND the A operand of
 //         D2 += X_{b+1}[:, j] x W1_{b+1}[:, j]   -> conv1 of the NEXT block accumulates in TMEM columns [256,512)
-//       D2 epilogue: T1_{b+1} = ReLU(D2 + shift1) -> staging set T -> TMA store + release of counter[b+1]
+//       D2 epilogue: T1_{b+1} = ReLU(D2 + shift1) -> staging set T -> TMA store group by group; counter[b+1][c] is
+//       released once the bulk store of group c has completed (bulk groups complete in order, so X_{b+1}, stored
+//       earlier, is in global memory too before the first of them)
 // so a block costs one halo exchange and its 1x1 convolutions never read their input from memory again.
 // P1 (once): T1_0 = conv1 of the first block, a plain GEMM over X_0.
 //
+// Counters: [tiles_n][nblocks + 1][4] (image group, block, 64-channel chunk) + one exit counter; the last CTA to
+// leave re-arms them all to zero.  T1_b lives in the parity buffer n0 + (b & 1) * N, so T1_{b+1} overwrites T1_{b-1}.
+// That is safe: a tile stores T1_{b+1} only after its own conv2 of block b, whose halo loads (and the conv3 loads
+// behind them) the producer issues only after all four counter[b][c] have been acquired; and a neighbour releases ANY
+// counter[b][c] only after its D2 epilogue of block b-1, which waits on an MMA commit issued after every conv2 MMA of
+// block b-1, i.e. after every halo load of T1_{b-1} it made has landed.  All four counters of a block are acquired
+// even when a tile has no halo taps, which keeps this ordering (and the residual loads of X_b behind them) intact.
+// The acquiring is done by the counter watcher (warp 3), which hands each counter[b][c] to the producer through a
+// shared-memory barrier: a global round trip per chunk inside the producer would stall the ring's feed.
+//
+// The epilogue reads the BatchNorm shifts from shared memory: at the start of each block the epilogue warps copy that
+// block's shift2 / shift3 and the next block's shift1 (6 KB) there while conv2 runs.  Read from global memory, every
+// 64-column group began with an L2 round trip for a line no warp of the SM had touched yet.
+//
 // Warp roles (384 threads): 0 = TMA producer, 1 = MMA issuer (leader CTA), 2 = TMEM alloc + store thread,
-// 3 = idle, 4..11 = epilogue.
+// 3 = counter watcher, 4..11 = epilogue.
 #include <cuda.h>
 #include <stdlib.h>
 
@@ -37,6 +58,7 @@ constexpr uint32_t kBcBuf = 16384;         // staging buffer: 128 px x 64 ch
 constexpr int kBcP = 256;                  // planes
 constexpr int kBcC = 1024;                 // 4 * planes
 constexpr int kBcNT = 8;                   // conv3 N-tiles of 128
+constexpr int kBcShifts = kBcP + kBcC + kBcP;     // shift2[b], shift3[b], shift1[b+1] staged in shared memory
 constexpr long long kBcSpinLimit = 6000000000LL;
 
 struct BcParams {
@@ -49,7 +71,7 @@ struct BcParams {
   const float* shift1;        // [nblocks][256]
   const float* shift2;        // [nblocks][256]
   const float* shift3;        // [nblocks][1024]
-  unsigned int* counters;     // [tiles_n][nblocks + 1] + exit counter
+  unsigned int* counters;     // [tiles_n][nblocks + 1][4] + exit counter
   int fmt;
   unsigned long long* dbg;
 };
@@ -118,7 +140,8 @@ __global__ void __launch_bounds__(kBcThreads, 1)
   const uint32_t stgT = smem_base + p.slots * kBcSlotBytes;       // 4 buffers: t1 / t2 tiles (256 channels)
   const uint32_t stgO = stgT + 4 * kBcBuf;                         // 2 buffers: one 128-channel N-tile of the block output
   const uint32_t ident = stgO + 2 * kBcBuf;                        // identity B tile for the residual MMAs (8 KB)
-  const uint32_t bars = ident + 8192u;
+  const uint32_t shf = ident + 8192u;                              // BatchNorm shifts of one block (6 KB), see stage_shifts
+  const uint32_t bars = shf + 4u * kBcShifts;
   auto full_bar = [&](int s) { return bars + 8u * s; };
   auto empty_bar = [&](int s) { return bars + 8u * (kBcMaxSlots + s); };
   const uint32_t b0 = bars + 8u * (2 * kBcMaxSlots);
@@ -131,7 +154,8 @@ __global__ void __launch_bounds__(kBcThreads, 1)
   auto availO = [&](int g) { return b0 + 8u * (18 + g); };         // [2]
   auto readyO = [&](int g) { return b0 + 8u * (20 + g); };         // [2]
   auto s2readyO = [&](int g) { return b0 + 8u * (22 + g); };       // [2]
-  const uint32_t tmem_slot = b0 + 8u * 24;
+  auto haloT = [&](int c) { return b0 + 8u * (24 + c); };          // [4] counter[b][c] acquired, one phase per block
+  const uint32_t tmem_slot = b0 + 8u * 28;
   volatile uint32_t* tmem_slot_ptr = reinterpret_cast<volatile uint32_t*>(smem_al + (tmem_slot - smem_base));
 
   const int warp = threadIdx.x >> 5;
@@ -143,7 +167,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
   const int pair = cluster_id / per, tt = cluster_id % per;
   const int tn = 2 * pair + static_cast<int>(crank);
   const int n0 = tn * p.bn, h0 = (tt / p.tiles_w) * p.bh, w0 = (tt % p.tiles_w) * p.bw;
-  unsigned int* ctr = p.counters + static_cast<size_t>(tn) * (p.nblocks + 1);
+  unsigned int* ctr = p.counters + static_cast<size_t>(tn) * (p.nblocks + 1) * 4;     // [block][chunk]
   const int nb = p.nblocks;
   if (threadIdx.x == 0) BC_STAMP(0);
 
@@ -173,6 +197,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
       mbar_init(readyO(g), kBcEpiThreads / 32);
       mbar_init(s2readyO(g), 2 * (kBcEpiThreads / 32));
     }
+    for (int c = 0; c < 4; ++c) mbar_init(haloT(c), 1);
     fence_barrier_init();
   }
   if (warp == 2) tmem_alloc_2cta(tmem_slot, 512);
@@ -252,22 +277,22 @@ __global__ void __launch_bounds__(kBcThreads, 1)
       const int wrow = (b * 9 + 4) * kBcP + static_cast<int>(crank) * 128;
       issue_b2(&tmW2, 0, wrow);
       issue_b2(&tmW2, 128, wrow);
-      // the other taps read halo tiles of T1_b: every tile of this image group has stored it
-      if (lane == 0) bc_wait_counter(ctr + b, per);
-      __syncwarp();
-      bc_fence_async();
-      if (lane == 0 && b < 3) BC_STAMP(2 + b);
+      // then the halo taps, chunk-major: those of chunk c read chunk c of T1_b's halo tiles, which every tile of this
+      // image group has stored once the counter watcher passes haloT(c)
       int kh_lo, kh_hi, kw_lo, kw_hi;
       bc_taps(p.dil, h0, p.bh, p.H, kh_lo, kh_hi);
       bc_taps(p.dil, w0, p.bw, p.W, kw_lo, kw_hi);
       const int tnn = n0 + (b & 1) * p.N;
-      for (int kh = kh_lo; kh <= kh_hi; ++kh)
-        for (int kw = kw_lo; kw <= kw_hi; ++kw) {
-          if (kh == 1 && kw == 1) continue;
-          for (int chunk = 0; chunk < kBcP / 64; ++chunk)
+      for (int chunk = 0; chunk < kBcP / 64; ++chunk) {
+        mbar_wait(haloT(chunk), static_cast<uint32_t>(b) & 1u);
+        bc_fence_async();
+        for (int kh = kh_lo; kh <= kh_hi; ++kh)
+          for (int kw = kw_lo; kw <= kw_hi; ++kw) {
+            if (kh == 1 && kw == 1) continue;
             issue(&tmT, chunk * 64, w0 + (kw - 1) * p.dil, h0 + (kh - 1) * p.dil, tnn, &tmW2, chunk * 64,
                   (b * 9 + kh * 3 + kw) * kBcP + static_cast<int>(crank) * 128);
-        }
+          }
+      }
       // P3: per conv3 N-tile one slot with its four 64-row filter chunks and one slot with the two residual chunks of
       // X_b; per next-conv1 slice one slot with its two filter chunks - in the order the MMA issuer consumes them
       const CUtensorMap* xmap = (b & 1) ? &tmXb : &tmXa;
@@ -360,6 +385,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
             for (int k = 0; k < 4; ++k) umma_f16_2cta(tmem_base, ad + 2u * k, bd + 2u * k, p.idesc256, (c | k) ? 1u : 0u);
           }
           umma_commit_2cta_mc(empty_bar(slot), 3);
+          if (s2 == 0 && b < 3) BC_STAMP(23 + b);
           if (s2 == 1) {
             for (int g = 0; g < 4; ++g) umma_commit_2cta_mc(availT(g), 3);       // t1 tile consumed
             if (nkb == 0) {
@@ -371,6 +397,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
         __syncwarp();
         advance();
       }
+      // the halo taps, chunk-major (chunk 0's eight taps first): the order the producer loads them in
       for (int kb = 0; kb < nkb; ++kb) {
         mbar_wait(full_bar(slot), phase);
         tcgen05_after_thread_sync();
@@ -380,6 +407,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
 #pragma unroll
           for (int k = 0; k < 4; ++k) umma_f16_2cta(tmem_base, ad + 2u * k, bd + 2u * k, p.idesc256, 1u);
           umma_commit_2cta_mc(empty_bar(slot), 3);
+          if (kb == 0 && b < 3) BC_STAMP(26 + b);
           if (kb == nkb - 1) {
             umma_commit_2cta_mc(tfull_bar(0), 3);
             umma_commit_2cta_mc(tfull_bar(1), 3);
@@ -396,21 +424,21 @@ __global__ void __launch_bounds__(kBcThreads, 1)
         wait_acc(h);
         tcgen05_after_thread_sync();
         const uint32_t tacc = tmem_base + static_cast<uint32_t>(h) * 128u;
-        if (j == 0)
-          for (int c = 0; c < 4; ++c) mbar_wait(s2readyT(c), 1u);     // t2 (T use 2b+1: odd parity) staged in both CTAs
         // slot 1: the four 64-row filter chunks of this N-tile; A = the staged t2 tile
         mbar_wait(full_bar(slot), phase);
-        tcgen05_after_thread_sync();
-        if (elect_one()) {
-          for (int c = 0; c < 4; ++c) {
+        for (int c = 0; c < 4; ++c) {
+          // N-tile 0: K-chunk c as soon as t2 group c (T use 2b+1: odd parity) is staged in both CTAs
+          if (j == 0) mbar_wait(s2readyT(c), 1u);
+          tcgen05_after_thread_sync();
+          if (elect_one()) {
             const uint64_t ad = tdesc0 + static_cast<uint64_t>((kBcBuf >> 4) * c);
             const uint64_t bd = adesc0 + static_cast<uint64_t>(slot_step * slot) + static_cast<uint64_t>((8192u >> 4) * c);
 #pragma unroll
             for (int k = 0; k < 4; ++k) umma_f16_2cta(tacc, ad + 2u * k, bd + 2u * k, p.idesc128, (c | k) ? 1u : 0u);
+            if (c == 3) umma_commit_2cta_mc(empty_bar(slot), 3);
           }
-          umma_commit_2cta_mc(empty_bar(slot), 3);
+          __syncwarp();
         }
-        __syncwarp();
         advance();
         // slot 2: residual  D[:, c*64 .. c*64+63] += X_b tile chunk x I   (exact: products with 1.0)
         mbar_wait(full_bar(slot), phase);
@@ -466,19 +494,32 @@ __global__ void __launch_bounds__(kBcThreads, 1)
   } else if (threadIdx.x == 64) {
     // ===================== store thread =====================
     uint32_t nT = 0, nO = 0;
+    // group g of T1_{b1} is in global memory: its staging buffer is free (the other arrival: the centre-tap MMAs of
+    // conv2) and counter[b1][g] lets the neighbours load its halo
+    auto publish = [&](int b1, int g) {
+      mbar_arrive(availT(g));
+      bc_fence_async();
+      __threadfence();
+      bc_red_release(ctr + b1 * 4 + g, 1u);
+    };
+    // T1_{b1} group by group.  Bulk groups complete in order: once the store of group g is complete, so is every
+    // store committed before it (the X_{b1} tile among them, which block b1 reads back as its residual)
+    auto store_t1 = [&](int b1) {
+      for (int g = 0; g < 4; ++g) {
+        mbar_wait(readyT(g), nT & 1u);
+        tma_store_5d(&tmT, stgT + g * kBcBuf, g * 64, w0, 0, h0, n0 + (b1 & 1) * p.N);
+        tma_store_commit();
+        if (g > 0) {
+          tma_store_wait_all<1>();
+          publish(b1, g - 1);
+        }
+      }
+      tma_store_wait_all<0>();
+      publish(b1, 3);
+      ++nT;
+    };
     // P1: T1_0
-    for (int g = 0; g < 4; ++g) {
-      mbar_wait(readyT(g), nT & 1u);
-      tma_store_5d(&tmT, stgT + g * kBcBuf, g * 64, w0, 0, h0, n0);
-      tma_store_commit();
-    }
-    tma_store_wait_read<0>();
-    for (int g = 0; g < 4; ++g) mbar_arrive(availT(g));      // the second arrival: centre-tap MMAs of the next conv2
-    tma_store_wait_all<0>();
-    bc_fence_async();
-    __threadfence();
-    bc_red_release(ctr + 0, 1u);
-    ++nT;
+    store_t1(0);
     for (int b = 0; b < nb; ++b) {
       const bool next = b + 1 < nb;
       // t2 stays on chip: only the bookkeeping arrival (the second one is the MMA commit after the last conv3 tile)
@@ -501,22 +542,19 @@ __global__ void __launch_bounds__(kBcThreads, 1)
         }
         ++nO;
       }
-      if (next) {
-        for (int g = 0; g < 4; ++g) {
-          mbar_wait(readyT(g), nT & 1u);
-          tma_store_5d(&tmT, stgT + g * kBcBuf, g * 64, w0, 0, h0, n0 + ((b + 1) & 1) * p.N);
-          tma_store_commit();
-        }
-        tma_store_wait_read<0>();
-        for (int g = 0; g < 4; ++g) mbar_arrive(availT(g));
-        tma_store_wait_all<0>();       // X_{b+1} and T1_{b+1} of this tile are in global memory
-        bc_fence_async();
-        __threadfence();
-        bc_red_release(ctr + b + 1, 1u);
-        ++nT;
-      }
+      if (next) store_t1(b + 1);
     }
     tma_store_wait_all<0>();
+  } else if (threadIdx.x == 96) {
+    // ===================== counter watcher =====================
+    // acquires counter[b][c] and passes it to the producer through haloT(c), so that the producer's ring feed never
+    // waits for a global round trip.  It cannot run a phase ahead: counter[b+1][c] needs this tile's T1_{b+1}, i.e.
+    // its conv2 of block b, i.e. the producer past every haloT wait of block b.
+    for (int b = 0; b < nb; ++b)
+      for (int c = 0; c < 4; ++c) {
+        bc_wait_counter(ctr + b * 4 + c, per);
+        mbar_arrive(haloT(c));
+      }
   } else if (warp >= kBcEpiWarp0) {
     // ===================== epilogue (8 warps) =====================
     const int ew = warp - kBcEpiWarp0;
@@ -528,22 +566,37 @@ __global__ void __launch_bounds__(kBcThreads, 1)
     const uint32_t row7 = static_cast<uint32_t>(row) & 7u;
     const uint32_t tlane = static_cast<uint32_t>(quarter * 32) << 16;
     uint32_t nT = 0, nO = 0;
-    uint32_t use[2] = {0u, 0u};
+    uint32_t fullpar = 0u;        // bit h: parity of the next tfull_bar(h) phase
+    float* const shs = reinterpret_cast<float*>(smem_al + (shf - smem_base));
+    auto release = [&](int h) {
+      if (lane == 0) {
+        if (crank == 0) mbar_arrive(tempty_bar(h));
+        else mbar_arrive_remote(tempty_bar(h), 0u);
+      }
+    };
 
     // `groups` x 64 accumulator columns from tmem_col0 -> ReLU(acc + shift) -> 16-bit -> staging buffers stg[g].
-    // setO: the O set (2 buffers) instead of the T set (4); second: also hand them to the MMA issuer (A operand).
-    auto epilogue = [&](uint32_t tmem_col0, int groups, const float* sh, bool setO, bool second) {
+    // setO: the O set (2 buffers) instead of the T set (4); second: also hand them to the MMA issuer (A operand);
+    // release0: hand accumulator half 0 (groups 0-1) back to the MMA issuer as soon as group 1 is in registers.
+    // sho: offset of the shifts in the staged table (shared memory: a global load here would put an L2 round trip in
+    // front of every 64-column group)
+    auto epilogue = [&](uint32_t tmem_col0, int groups, int sho, bool setO, bool second, bool release0) {
       uint32_t r[32];
       const uint32_t taddr = tmem_col0 + tlane + static_cast<uint32_t>(half * 32);
       const uint32_t nuse = setO ? nO : nT;
       tmem_ld_32x32b_x32(taddr, r);
       for (int g = 0; g < groups; ++g) {
-        const float4* s4 = reinterpret_cast<const float4*>(sh + g * 64 + half * 32);
+        const float4* s4 = reinterpret_cast<const float4*>(shs + sho + g * 64 + half * 32);
         float v[32];
         tmem_ld_wait();
+        if (release0 && g == 1) {       // every load of half 0 has completed; the load of group 2 is not issued yet
+          tcgen05_before_thread_sync();
+          __syncwarp();
+          release(0);
+        }
 #pragma unroll
         for (int j4 = 0; j4 < 8; ++j4) {
-          const float4 h4 = __ldg(s4 + j4);
+          const float4 h4 = s4[j4];
           v[4 * j4 + 0] = __uint_as_float(r[4 * j4 + 0]) + h4.x;
           v[4 * j4 + 1] = __uint_as_float(r[4 * j4 + 1]) + h4.y;
           v[4 * j4 + 2] = __uint_as_float(r[4 * j4 + 2]) + h4.z;
@@ -576,34 +629,43 @@ __global__ void __launch_bounds__(kBcThreads, 1)
       if (setO) ++nO; else ++nT;
     };
     auto wait_full = [&](int h) {
-      mbar_wait(tfull_bar(h), use[h] & 1u);
-      ++use[h];
+      mbar_wait(tfull_bar(h), (fullpar >> h) & 1u);
+      fullpar ^= 1u << h;
     };
-    auto release = [&](int h) {
-      if (lane == 0) {
-        if (crank == 0) mbar_arrive(tempty_bar(h));
-        else mbar_arrive_remote(tempty_bar(h), 0u);
+    // The shifts block b's epilogues use: [0,256) shift2[b], [256,1280) shift3[b], [1280,1536) shift1[b+1] (the T1
+    // epilogue of the next block); b = -1 stages only shift1[0].  Copied while the epilogue warps wait for conv2, once
+    // every epilogue warp is done with the previous block's table.
+    auto stage_shifts = [&](int b) {
+      asm volatile("bar.sync 1, %0;" ::"n"(kBcEpiThreads) : "memory");
+      for (int e = 4 * etid; e < kBcShifts; e += 4 * kBcEpiThreads) {
+        const float* src = e < kBcP ? p.shift2 + b * kBcP + e
+                           : e < kBcP + kBcC ? p.shift3 + b * kBcC + (e - kBcP)
+                                             : p.shift1 + (b + 1) * kBcP + (e - kBcP - kBcC);
+        if ((e < kBcP + kBcC && b < 0) || (e >= kBcP + kBcC && b + 1 >= nb)) continue;
+        *reinterpret_cast<float4*>(shs + e) = __ldg(reinterpret_cast<const float4*>(src));
       }
+      asm volatile("bar.sync 1, %0;" ::"n"(kBcEpiThreads) : "memory");
     };
     // ---- P1: T1_0 = ReLU(bn1(conv1(X_0))) ----
+    stage_shifts(-1);
     wait_full(0);
     wait_full(1);
     tcgen05_after_thread_sync();
-    epilogue(tmem_base, 4, p.shift1, false, true);
+    epilogue(tmem_base, 4, kBcP + kBcC, false, true, false);
     tcgen05_before_thread_sync();
     __syncwarp();
     release(0);
     release(1);
     for (int b = 0; b < nb; ++b) {
       const bool next = b + 1 < nb;
-      // ---- P2: t2 (stays on chip) ----
+      stage_shifts(b);
+      // ---- P2: t2 (stays on chip); half 0 goes back mid-epilogue, conv3 N-tile 0 writes only there ----
       wait_full(0);
       wait_full(1);
       tcgen05_after_thread_sync();
-      epilogue(tmem_base, 4, p.shift2 + b * kBcP, false, true);
+      epilogue(tmem_base, 4, 0, false, true, true);
       tcgen05_before_thread_sync();
       __syncwarp();
-      release(0);
       release(1);
       if (b < 3 && etid == 0) BC_STAMP(11 + b);
       // ---- P3: the block's output, 128 channels at a time ----
@@ -611,7 +673,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
         const int h = j & 1;
         wait_full(h);
         tcgen05_after_thread_sync();
-        epilogue(tmem_base + static_cast<uint32_t>(h) * 128u, 2, p.shift3 + b * kBcC + j * 128, true, next);
+        epilogue(tmem_base + static_cast<uint32_t>(h) * 128u, 2, kBcP + j * 128, true, next, false);
         tcgen05_before_thread_sync();
         __syncwarp();
         release(h);
@@ -621,7 +683,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
         // ---- T1_{b+1} = ReLU(bn1(conv1(X_{b+1}))) from the second accumulator ----
         mbar_wait(d2full_bar, b & 1u);
         tcgen05_after_thread_sync();
-        epilogue(tmem_d2, 4, p.shift1 + (b + 1) * kBcP, false, true);
+        epilogue(tmem_d2, 4, kBcP + kBcC, false, true, false);
         tcgen05_before_thread_sync();
         __syncwarp();
         if (lane == 0) {
@@ -643,7 +705,7 @@ __global__ void __launch_bounds__(kBcThreads, 1)
     tmem_dealloc_2cta(tmem_base, 512);
   }
   if (threadIdx.x == 0) {
-    const int n_ctr = p.tiles_n * (p.nblocks + 1);
+    const int n_ctr = p.tiles_n * (p.nblocks + 1) * 4;
     __threadfence();
     const unsigned int old = atomicAdd(p.counters + n_ctr, 1u);
     if (old == gridDim.x - 1) {
@@ -748,7 +810,8 @@ extern "C" int up_bneck_chain_supported(const UpBneckChainDesc* d) {
 extern "C" int64_t up_bneck_chain_workspace_bytes(const UpBneckChainDesc* d) {
   BcPlan pl;
   if (bc_plan(d, pl)) return -1;
-  return ((static_cast<int64_t>(pl.tiles_n) * (d->nblocks + 1) + 1) * 4 + 255) & ~static_cast<int64_t>(255);
+  // counters [tiles_n][nblocks + 1][4 chunks] + the exit counter, 4 bytes each
+  return ((static_cast<int64_t>(pl.tiles_n) * (d->nblocks + 1) * 4 + 1) * 4 + 255) & ~static_cast<int64_t>(255);
 }
 
 extern "C" int up_bneck_chain_fwd(const UpBneckChainDesc* d, const UpBneckChainWeights* w, void* xa, void* xb, void* t1,
@@ -777,7 +840,7 @@ extern "C" int up_bneck_chain_fwd(const UpBneckChainDesc* d, const UpBneckChainW
   p.tiles_n = pl.tiles_n;
   p.nblocks = d->nblocks;
   p.dil = d->dil;
-  const size_t fixed = 1024 + 6 * kBcBuf + 8192 + 8 * (2 * kBcMaxSlots + 24) + 16;
+  const size_t fixed = 1024 + 6 * kBcBuf + 8192 + 4 * kBcShifts + 8 * (2 * kBcMaxSlots + 28) + 16;
   int slots = static_cast<int>((di->max_smem - fixed) / kBcSlotBytes);
   if (slots > kBcMaxSlots) slots = kBcMaxSlots;
   UP_CHECK_ARG(slots >= 2, "up_bneck_chain_fwd: not enough shared memory");
