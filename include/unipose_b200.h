@@ -295,6 +295,29 @@ int up_pack_input_s2d(const float* x_nchw, void* y, int n, int h, int w, int dty
  * fused with the stem's input packing; a quarter of the host->device bytes of the fp32 NCHW path, identical bits. */
 int up_pack_input_u8_s2d(const uint8_t* x_nhwc, void* y, int n, int h, int w, int dtype, int64_t y_plane_stride,
                          int y_wpitch, int y_wpad_left, float mean, float std_, void* stream);
+/* Ragged batch of decoded uint8 HWC images (3 channels, any sizes) -> the network input, in one launch:
+ * cv2.resize(img, (out_w, out_h)) (utils/mpii_data.py:159-162, utils/lsp_lspet_data.py:211, penn_action_data.py),
+ * bit for bit OpenCV's 8-bit INTER_LINEAR path (11-bit fixed-point weights, the SIMD vertical rounding
+ * ((r0 >> 4) * b0 >> 16) + ((r1 >> 4) * b1 >> 16), (v + 2) >> 2; a source of exactly twice the target size takes
+ * cv2's 2x2 INTER_AREA average), then, where UpImageJob.flip is set, the mirror of Mytransforms.hflip
+ * (utils/Mytransforms.py:501-505: output column x takes resized column out_w - 1 - x).
+ *   jobs:      HOST copy of the table (validated, and sizes the launch); jobs_dev: the same n entries in device memory,
+ *              which the kernel reads.  Each `src` must stay valid until the launch has run on `stream`.
+ *   out_format UP_BF16 / UP_FP16 / UP_SPLIT: the normalised (x - mean) / std space-to-depth tensor of
+ *              up_pack_input_u8_s2d, same layout (y_plane_stride, y_wpitch, y_wpad_left) and same bits;
+ *              UP_RESIZE_OUT_U8: uint8 HWC [n, out_h, out_w, 3] (the resized images);
+ *              UP_RESIZE_OUT_F32: fp32 NCHW [n, 3, out_h, out_w], (x - mean) / std (Mytransforms.normalize).
+ *   out_h, out_w: multiples of 16 (the stem's requirement). */
+enum { UP_RESIZE_OUT_U8 = 8, UP_RESIZE_OUT_F32 = 9 };
+typedef struct UpImageJob {
+  const uint8_t* src;     /* row 0, column 0, channel 0 of the image, device memory */
+  int32_t h, w;           /* source size in pixels, both > 0 */
+  int32_t pitch;          /* bytes from one row to the next, >= 3 * w */
+  int32_t flip;           /* 1: mirror the resized image horizontally */
+} UpImageJob;
+int up_resize_pack_u8(const UpImageJob* jobs, const UpImageJob* jobs_dev, int n, int out_h, int out_w, int out_format,
+                      void* y, int64_t y_plane_stride, int y_wpitch, int y_wpad_left, float mean, float std_,
+                      void* stream);
 /* Ground-truth heat-maps on the device (utils/mpii_data.py:62-65,165-181; same code in lsp_lspet_data / bbc_data):
  * kpts fp32 [n,k,2] (x, y in input-image pixels) -> heat fp32 NCHW [n, k + background, h, w]: channel j+background
  * = exp(-((x - cx)^2 + (y - cy)^2) / 2 / sigma / sigma) in float64 with cx = int(kx) / stride (truncate_mode 1) or

@@ -11,6 +11,7 @@ from ctypes import POINTER, c_char_p, c_float, c_int, c_int32, c_int64, c_void_p
 from . import build as _build
 
 UP_BF16, UP_FP16, UP_SPLIT = 0, 1, 2
+UP_RESIZE_OUT_U8, UP_RESIZE_OUT_F32 = 8, 9
 UP_FLAG_RELU, UP_FLAG_RESIDUAL, UP_FLAG_OUT_NCHW_F32, UP_FLAG_STATS, UP_FLAG_PROJ = 1, 2, 4, 8, 16
 
 
@@ -48,6 +49,10 @@ class UpEpilogueJob(ctypes.Structure):
                 ("fold_scale", c_void_p), ("scale", c_void_p), ("shift", c_void_p),
                 ("eps", c_float), ("c_bn", c_int32), ("bias_len", c_int32), ("cout_real", c_int32), ("cout", c_int32),
                 ("fold_into_weights", c_int32), ("reserved", c_int32 * 2)]
+
+
+class UpImageJob(ctypes.Structure):
+    _fields_ = [("src", c_void_p), ("h", c_int32), ("w", c_int32), ("pitch", c_int32), ("flip", c_int32)]
 
 
 class UpWaspChainDesc(ctypes.Structure):
@@ -90,6 +95,7 @@ _SIGNATURES = {
     "up_bn_fold": [_P, _P, _P, _P, _F, _P, _P, _I, _I, _P],
     "up_pack_input_s2d": [_P, _P, _I, _I, _I, _I, _L, _I, _I, _P],
     "up_pack_input_u8_s2d": [_P, _P, _I, _I, _I, _I, _L, _I, _I, _F, _F, _P],
+    "up_resize_pack_u8": [POINTER(UpImageJob), _P, _I, _I, _I, _I, _P, _L, _I, _I, _F, _F, _P],
     "up_gaussian_labels": [_P, _P, _I, _I, _I, _I, _F, _F, _I, _I, _P],
     "up_nchw_f32_to_nhwc": [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _L, _P],
     "up_nhwc_to_nchw_f32": [_P, _P, _I, _I, _I, _I, _I, _I, _I, _L, _P],

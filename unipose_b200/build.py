@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 LIB_DIR = os.path.join(_HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libunipose_b200.so")
-SOURCES = ["conv_tcgen05.cu", "conv_wgrad_tcgen05.cu", "wasp_chain.cu", "bneck_chain.cu", "bneck_tail.cu", "elementwise.cu", "video_eval.cu", "train.cu", "pack_multi.cu", "data_pipeline.cu", "c_api.cu"]
+SOURCES = ["conv_tcgen05.cu", "conv_wgrad_tcgen05.cu", "wasp_chain.cu", "bneck_chain.cu", "bneck_tail.cu", "elementwise.cu", "video_eval.cu", "train.cu", "pack_multi.cu", "data_pipeline.cu", "image_prep.cu", "c_api.cu"]
 HEADERS = ["up_ptx.cuh", "up_internal.h", "up_conv_host.h", os.path.join("..", "..", "include", "unipose_b200.h")]
 
 NVCC_FLAGS = [

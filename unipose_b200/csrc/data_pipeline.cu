@@ -9,25 +9,6 @@
 
 namespace up {
 
-template <int kMode>
-__device__ __forceinline__ void dp_store8(uint16_t* p, long long plane, const float (&v)[8]) {
-  uint32_t h[4], l[4];
-#pragma unroll
-  for (int e = 0; e < 4; ++e) {
-    if constexpr (kMode == 2) {
-      uint16_t h0, l0, h1, l1;
-      split_bf16(v[2 * e], h0, l0);
-      split_bf16(v[2 * e + 1], h1, l1);
-      h[e] = h0 | (static_cast<uint32_t>(h1) << 16);
-      l[e] = l0 | (static_cast<uint32_t>(l1) << 16);
-    } else {
-      h[e] = cvt_f32_to16<kMode>(v[2 * e]) | (static_cast<uint32_t>(cvt_f32_to16<kMode>(v[2 * e + 1])) << 16);
-    }
-  }
-  *reinterpret_cast<uint4*>(p) = make_uint4(h[0], h[1], h[2], h[3]);
-  if constexpr (kMode == 2) *reinterpret_cast<uint4*>(p + plane) = make_uint4(l[0], l[1], l[2], l[3]);
-}
-
 // one thread per space-to-depth pixel: reads two rows x 6 bytes (2 pixels x 3 channels), writes 16 channels (12 real,
 // order (ph, pw, c) as up_pack_input_s2d)
 template <int kMode>
@@ -65,8 +46,8 @@ __global__ void pack_input_u8_s2d_kernel(const uint8_t* __restrict__ x, uint16_t
     }
   }
   uint16_t* o = y + ((static_cast<long long>(b) * hq + yq) * wpitch + xq + wpad) * 16;
-  dp_store8<kMode>(o, plane, v0);
-  dp_store8<kMode>(o + 8, plane, v1);
+  store8_16<kMode>(o, plane, v0);
+  store8_16<kMode>(o + 8, plane, v1);
 }
 
 // one thread per (image, pixel): all K joints + the background channel

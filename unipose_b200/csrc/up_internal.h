@@ -112,4 +112,25 @@ __device__ __forceinline__ void split_bf16(float x, uint16_t& hi, uint16_t& lo) 
 
 inline int fmt_of_dtype(int dtype) { return dtype == UP_FP16 ? 0 : 1; }
 
+// Eight fp32 values -> one 16-byte store of 16-bit values; kMode 0 = fp16, 1 = bf16, 2 = bf16 hi at p and lo at
+// p + plane (UP_SPLIT).  The stem's space-to-depth input writers (data_pipeline.cu, image_prep.cu) share it.
+template <int kMode>
+__device__ __forceinline__ void store8_16(uint16_t* p, long long plane, const float (&v)[8]) {
+  uint32_t h[4], l[4];
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    if constexpr (kMode == 2) {
+      uint16_t h0, l0, h1, l1;
+      split_bf16(v[2 * e], h0, l0);
+      split_bf16(v[2 * e + 1], h1, l1);
+      h[e] = h0 | (static_cast<uint32_t>(h1) << 16);
+      l[e] = l0 | (static_cast<uint32_t>(l1) << 16);
+    } else {
+      h[e] = cvt_f32_to16<kMode>(v[2 * e]) | (static_cast<uint32_t>(cvt_f32_to16<kMode>(v[2 * e + 1])) << 16);
+    }
+  }
+  *reinterpret_cast<uint4*>(p) = make_uint4(h[0], h[1], h[2], h[3]);
+  if constexpr (kMode == 2) *reinterpret_cast<uint4*>(p + plane) = make_uint4(l[0], l[1], l[2], l[3]);
+}
+
 }  // namespace up

@@ -269,12 +269,16 @@ class ResNet(PlanModule):
     def _input_channels_pad(self, idx, c):
         return 16
 
-    def _emit_image(self, b, x_static):
+    def _emit_image(self, b, x_static, s2d_shape=None):
         """x_static: fp32 NCHW [n,3,h,w] (the reference's input) or uint8 NHWC [n,h,w,3] (raw images; normalised
-        (x-128)/256 while packing, utils/mpii_data.py:184-185)."""
+        (x-128)/256 while packing, utils/mpii_data.py:184-185).  x_static None with s2d_shape = (n, h, w): the plan
+        starts at the stem convolution and the caller writes its space-to-depth input, b.plan.s2d_input, before each
+        run (unipose.forward_images)."""
         from .... import ops
-        u8 = x_static.dtype == torch.uint8
-        if u8:
+        u8 = x_static is not None and x_static.dtype == torch.uint8
+        if x_static is None:
+            n, h, w = s2d_shape
+        elif u8:
             n, h, w, _ = x_static.shape
         else:
             n, _, h, w = x_static.shape
@@ -286,7 +290,9 @@ class ResNet(PlanModule):
         # activation row the TMA fetches is 128 aligned bytes and is shared by 4 outputs.
         ws = w // 8
         x2 = b.act(n, h // 2, ws + 1, 64, zero=True)
-        if u8:
+        if x_static is None:
+            b.plan.s2d_input = x2
+        elif u8:
             b.add(lambda x_static=x_static, x2=x2: ops.pack_input_u8_s2d(x_static, x2, wpad_left=2), "pack_input_u8_s2d")
         else:
             b.add(lambda x_static=x_static, x2=x2: ops.pack_input_s2d(x_static, x2, wpad_left=2), "pack_input_s2d")

@@ -28,13 +28,18 @@ class unipose(PlanModule):
             self.freeze_bn()
 
     # ------------------------------------------------------------------------------------------
-    def _build_plan(self, shape, device, u8=False):
+    def _build_plan(self, shape, device, u8=False, s2d=False):
         plan = engine.Plan(device, self._precision())
         b = plan.builder
-        st = plan.static_input(shape, dtype=torch.uint8 if u8 else torch.float32)
-        if u8:
-            shape = (shape[0], 3, shape[1], shape[2])
-        x, low = self.backbone._emit_image(b, st)
+        if s2d:
+            # shape = (n, 3, h, w): no input tensor, the plan starts at the stem (forward_images fills plan.s2d_input)
+            st = None
+            x, low = self.backbone._emit_image(b, None, s2d_shape=(shape[0], shape[2], shape[3]))
+        else:
+            st = plan.static_input(shape, dtype=torch.uint8 if u8 else torch.float32)
+            if u8:
+                shape = (shape[0], 3, shape[1], shape[2])
+            x, low = self.backbone._emit_image(b, st)
         x = self.wasp._emit(b, x)
         heat = self.decoder._emit(b, x, low)
         if self.stride != 8:   # model/unipose.py:31-32
@@ -68,6 +73,31 @@ class unipose(PlanModule):
             raise NotImplementedError("forward_uint8 is an inference entry point (call .eval())")
         self._bn_eval_only()
         return self.plan_for(images).run(images.contiguous())[0].clone()
+
+    def forward_images(self, images, size=368, shapes=None):
+        """Inference on a ragged batch of decoded uint8 HWC images of any sizes (a list of [h, w, 3] CUDA tensors, or
+        one packed buffer with `shapes`, see data.ImageBatch): the reference's cv2.resize(img, (368, 368))
+        (utils/mpii_data.py:159-162) runs on the device, bit for bit, and writes the normalised space-to-depth input
+        of the stem directly; the result equals forward_uint8(cv2-resized batch) bit for bit.  The resize is one
+        launch on the current stream just before the graph replay of a plan keyed by (n, size, precision, device):
+        ragged source addresses change every call, so it is not part of the captured graph."""
+        from .. import data
+        if self.training:
+            raise NotImplementedError("forward_images is an inference entry point (call .eval())")
+        batch = data.ImageBatch(images, shapes)
+        s_h, s_w = data._out_size(size)
+        dev = next(self.parameters()).device
+        if batch.device != dev:
+            raise RuntimeError("unipose_b200: parameters on %s but images on %s (call .cuda())" % (dev, batch.device))
+        self._bn_eval_only()
+        key = ("images", batch.n, s_h, s_w, self._precision(), batch.device.index, self.stride)
+        plan = self._plans.get(key)
+        if plan is None:
+            plan = self._build_plan((batch.n, 3, s_h, s_w), batch.device, s2d=True)
+            self._plans[key] = plan
+        with torch.cuda.device(batch.device):
+            data.resize_into_s2d(batch, plan.s2d_input, (s_h, s_w), wpad_left=2)
+            return plan.run()[0].clone()
 
     def forward(self, input):
         self._check_inputs([input])
